@@ -17,6 +17,7 @@ two lane observations), one engine replica per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA engine
   python bench.py --impl reference [...]                         # reference CPU engine, host cores (rank 0 only)
+  python bench.py [...] --dump-outputs DIR                       # + the last timed step's results as DIR/<name>.npy
 
 Prints ONE JSON line on rank 0 (task contract): value / e2e / roofline / cpu_baseline / clocks / gpu_launches, plus
 `parity_check`: the sum of get_vehicle_count() over the timed steps of this run next to the same sum taken from the
@@ -74,6 +75,10 @@ def parse_args():
     p.add_argument("--multi", default="weak", choices=["weak", "sharded", "strong", "replicas"],
                    help="N>1, see the module docstring ('sharded' = 'weak')")
     p.add_argument("--clock-ms", type=int, default=50, help="nvidia-smi sampling period (0 = off)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps write what the last of them computed, as a caller of cityflow.Engine receives "
+                        "it, to DIR/<name>.npy (float64, at most 64 MB in all): identical arguments give identical inputs, so "
+                        "two builds can be compared output for output")
     p.add_argument("--profile-steps", type=int, default=0,
                    help="ncu mode: after prefill+warmup run this many steps between cudaProfilerStart/Stop and exit "
                         "(use with ncu --profile-from-start off)")
@@ -283,6 +288,49 @@ def run_reference_arm(args):
     print(json.dumps(line))
 
 
+DUMP_VEHICLES_MAX = 1 << 21   # vehicle arrays above this length are dumped as a fixed, seeded sample (2 x 16 MB)
+
+
+def write_outputs(directory, arrays):
+    """--dump-outputs: one float64 DIR/<name>.npy per array."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
+def engine_outputs(eng, ranks, sharded):
+    """The results of the step just taken as a caller of cityflow.Engine receives them: the vehicle count, per-lane vehicle
+    and waiting counts in lane_ids() order, and every running vehicle's speed and distance in the order of its id (all
+    ranks of a sharded run call this: the lane getters are collective, each rank reports the vehicles of its strip)."""
+    import numpy as np
+    out = {"vehicle_count": eng.get_vehicle_count()}
+    lanes = eng.lane_ids()
+    cnt, wait = eng.get_lane_vehicle_count(), eng.get_lane_waiting_vehicle_count()
+    out["lane_vehicle_count"] = [cnt[k] for k in lanes]
+    out["lane_waiting_vehicle_count"] = [wait[k] for k in lanes]
+    speed, distance = eng.get_vehicle_speed(), eng.get_vehicle_distance()
+    if sharded:
+        parts = [None] * ranks.world if ranks.rank == 0 else None
+        ranks.dist.gather_object((speed, distance), parts, dst=0)
+        if ranks.rank != 0:
+            return None
+        speed, distance = {}, {}
+        for sp, di in parts:
+            speed.update(sp)
+            distance.update(di)
+    ids = sorted(speed)
+    pick = np.arange(len(ids))
+    if len(ids) > DUMP_VEHICLES_MAX:
+        pick = np.sort(np.random.default_rng(0).choice(len(ids), DUMP_VEHICLES_MAX, replace=False))
+        out["vehicle_sample_index"] = pick
+    out["vehicle_speed"] = [speed[ids[i]] for i in pick]
+    out["vehicle_distance"] = [distance[ids[i]] for i in pick]
+    return out
+
+
 # ----------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -374,6 +422,10 @@ def run_ours(args):
     e2e_s = time.perf_counter() - t0
     barrier()
     m_hi = sampler.mark() if rank == 0 else 0
+    if args.dump_outputs:   # the last timed step: the end of the e2e loop (the kernel-timing pass below is untimed)
+        outputs = engine_outputs(eng, ranks, sharded)
+        if rank == 0:
+            write_outputs(args.dump_outputs, outputs)
     h2d1, d2h1 = eng.transfer_bytes()
     host_gen_ms, host_enq_ms = eng.host_times()
     # sharded: get_vehicle_count() already is the network-wide count on every rank
@@ -567,6 +619,11 @@ def run_ours_rl(args, ranks, sampler):
     torch.cuda.synchronize()
     eng.synchronize()
     dev_s = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:   # the last timed step of the device-resident loop: its actions and what it left
+        actions = votes.view(n_int, 8).argmax(1)
+        obs.refresh()
+        write_outputs(args.dump_outputs, {"tl_phases": actions.cpu(), "lane_vehicle_count": cnt.cpu(), "lane_waiting_vehicle_count": wait.cpu(),
+                                          "lane_speed_sum": obs.speed_sum.cpu(), "vehicle_steps": int(vs_dev)})
     ranks.barrier()
     m_hi = sampler.mark() if rank == 0 else 0
     sec = ranks.max(r["seconds"])

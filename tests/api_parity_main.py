@@ -5,102 +5,109 @@ getter, every step: the dicts of get_lane_vehicle_count / get_lane_waiting_vehic
 get_vehicle_distance (exact floats), the lists of get_vehicles (running and all) and of get_lane_vehicles (order on the
 lane included), get_vehicle_info's string dict, get_leader, times, and the same exceptions.  TEST INFRASTRUCTURE.
 
+The reference's side is pinned (tests/golden/reference/api_transcript.json, recorded by `tests/refpin.py api_transcript`):
+a digest of every call's result (tests/refpin.py canonical(): numbers as the bits of a double) per ten steps.
+
 Run as a script (`python tests/api_parity_main.py <config.json> <steps>`) it prints "OK ..." -- the CPU suite does that
 in a child process whose PYTHONPATH puts the emulated-device build of the module first (tests/test_cpu.py); the GPU suite
 calls compare_with_reference() in-process with the real module."""
+import hashlib
 import json
 import os
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GROUP = 10   # steps per pinned digest
 
 
-def compare_with_reference(ours_mod, ref_mod, cfg: str, steps: int) -> dict:
-    ref = ref_mod.Engine(cfg, thread_num=1)
-    eng = ours_mod.Engine(cfg, thread_num=1)
+def transcript(mod, cfg: str, steps: int):
+    """Runs the script on a `mod.Engine`; yields (step, the result of every call made in that step, counters)."""
+    eng = mod.Engine(cfg, thread_num=1)
     c = json.load(open(cfg))
     net = json.load(open(c["dir"] + c["roadnetFile"]))
     real = [i["id"] for i in net["intersections"] if not i["virtual"]]
     flows = json.load(open(c["dir"] + c["flowFile"]))
     some_route = flows[3]["route"]
     stats = dict(steps=0, infos=0, leaders=0, custom=0, rerouted_ok=0, rerouted_no=0, vehicles=0)
+    out = []
 
-    def same(name, *args, **kw):
-        a, b = getattr(ref, name)(*args, **kw), getattr(eng, name)(*args, **kw)
-        assert a == b, (name, args, stats["steps"], _first_difference(a, b))
-        return a
-
-    def both(name, *args, **kw):
-        """a call that changes state: same return value or the same kind of exception"""
-        out = []
-        for e in (ref, eng):
-            try:
-                out.append(("ok", getattr(e, name)(*args, **kw)))
-            except Exception as ex:   # noqa: BLE001  (pybind maps std::runtime_error to RuntimeError in both)
-                out.append(("raised", type(ex).__name__))
-        assert out[0] == out[1], (name, args, out)
-        return out[0]
+    def call(name, *args, **kw):
+        """the result, or the kind of exception (pybind maps std::runtime_error to RuntimeError in both modules)"""
+        try:
+            r = ("ok", getattr(eng, name)(*args, **kw))
+        except Exception as ex:   # noqa: BLE001
+            r = ("raised", type(ex).__name__)
+        out.append((name, r))
+        return r
 
     for s in range(1, steps + 1):
         stats["steps"] = s
+        out = []
         if s % 10 == 1 and c.get("rlTrafficLight"):
             for k, i in enumerate(real):
-                both("set_tl_phase", i, (s // 10 + k) % 8)
+                call("set_tl_phase", i, (s // 10 + k) % 8)
         if s in (40, 41, 150):
-            both("push_vehicle", {"speed": 3.0, "length": 6.5, "maxSpeed": 12.0} if s != 41 else {}, some_route)
+            call("push_vehicle", {"speed": 3.0, "length": 6.5, "maxSpeed": 12.0} if s != 41 else {}, some_route)
         if s == 120:
-            both("set_random_seed", 77)
+            call("set_random_seed", 77)
         if s == 200:
-            both("reset", seed=False)
-        running = same("get_vehicles")
+            call("reset", seed=False)
+        running = call("get_vehicles")[1]
         if s % 25 == 3:
             for vid in running[:: max(1, len(running) // 5)]:
-                both("set_vehicle_speed", vid, 0.5 * ref.get_vehicle_speed()[vid])
+                call("set_vehicle_speed", vid, 0.5 * eng.get_vehicle_speed()[vid])
                 stats["custom"] += 1
-            both("set_vehicle_speed", "flow_999999_0", 1.0)     # unknown vehicle: both raise
+            call("set_vehicle_speed", "flow_999999_0", 1.0)     # unknown vehicle: raises
         if s % 30 == 7:
             for j, vid in enumerate(running[1:: max(1, len(running) // 9)]):
                 target = flows[(s + j) % len(flows)]["route"][-1:] if j % 3 else ["no_such_road"]
-                ok = both("set_vehicle_route", vid, target)[1]
-                stats["rerouted_ok" if ok else "rerouted_no"] += 1
-        both("next_step")
-        assert same("get_vehicle_count") == len(same("get_vehicles"))
-        same("get_vehicles", include_waiting=True)
-        same("get_current_time")
-        same("get_lane_vehicle_count")
-        same("get_lane_waiting_vehicle_count")
-        same("get_lane_vehicles")
-        same("get_vehicle_speed")
-        same("get_vehicle_distance")
-        same("get_average_travel_time")
-        running = ref.get_vehicles()
+                ok = call("set_vehicle_route", vid, target)[1]
+                stats["rerouted_ok" if ok is True else "rerouted_no"] += 1
+        call("next_step")
+        assert call("get_vehicle_count")[1] == len(call("get_vehicles")[1])
+        call("get_vehicles", include_waiting=True)
+        call("get_current_time")
+        call("get_lane_vehicle_count")
+        call("get_lane_waiting_vehicle_count")
+        call("get_lane_vehicles")
+        call("get_vehicle_speed")
+        call("get_vehicle_distance")
+        call("get_average_travel_time")
+        running = eng.get_vehicles()
         for vid in running[:: max(1, len(running) // 6)]:
-            same("get_vehicle_info", vid)
-            same("get_leader", vid)
+            call("get_vehicle_info", vid)
+            call("get_leader", vid)
             stats["infos"] += 1
         stats["vehicles"] = len(running)
-    return stats
+        yield s, out, stats
 
 
-def _first_difference(a, b):
-    if isinstance(a, dict) and isinstance(b, dict):
-        for k in a:
-            if k not in b or a[k] != b[k]:
-                return (k, a[k], b.get(k))
-        return ("extra keys", sorted(set(b) - set(a))[:5])
-    if isinstance(a, list) and isinstance(b, list):
-        if len(a) != len(b):
-            return ("lengths", len(a), len(b))
-        for k, (x, y) in enumerate(zip(a, b)):
-            if x != y:
-                return (k, x, y)
-    return (a, b)
+def _digests(mod, cfg: str, steps: int):
+    """(steps of the group, digest of its calls' results, counters) per GROUP steps"""
+    import refpin
+    assert steps % GROUP == 0, steps
+    h = hashlib.sha256()
+    for s, out, stats in transcript(mod, cfg, steps):
+        h.update(refpin.canonical(out).encode())
+        if s % GROUP == 0:
+            yield [s - GROUP + 1, s], h.hexdigest()[:16], stats
+            h = hashlib.sha256()
+
+
+def record(ref_mod, cfg: str, steps: int) -> dict:
+    return {"group": GROUP, "entries": [{"steps": a, "digest": d} for a, d, _ in _digests(ref_mod, cfg, steps)]}
+
+
+def compare_with_reference(ours_mod, cfg: str, steps: int) -> dict:
+    import refpin
+    pin = refpin.load("api_transcript")
+    assert pin["group"] == GROUP and steps <= GROUP * len(pin["entries"]), (steps, len(pin["entries"]))
+    stats = None
+    for (a, d, stats), want in zip(_digests(ours_mod, cfg, steps), pin["entries"]):
+        assert a == want["steps"] and d == want["digest"], "steps %d..%d: some call returned another result than in the reference" % tuple(a)
+    return dict(stats)
 
 
 if __name__ == "__main__":
-    if ROOT not in sys.path:
-        sys.path.append(ROOT)          # for oracle.harness only; `import cityflow` is decided by what comes first
-    from oracle import harness as H
-    import cityflow
-    print("OK", json.dumps(compare_with_reference(cityflow, H.load_reference_module(), sys.argv[1], int(sys.argv[2]))),
-          "with", cityflow.__file__)
+    import cityflow          # first: whatever PYTHONPATH puts first
+    print("OK", json.dumps(compare_with_reference(cityflow, sys.argv[1], int(sys.argv[2]))), "with", cityflow.__file__)

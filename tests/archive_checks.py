@@ -1,6 +1,8 @@
 """Checks of the reference-schema JSON archive (Archive::dump archive.cpp:153-343, the file loader :345-550) shared by the
 CPU test (the real host engine over the emulated device, tests/test_cpu.py) and the GPU test (tests/test_gpu_zarchive.py).
-TEST INFRASTRUCTURE: the checker is the UNMODIFIED reference, compiled in oracle/_ref/refdump (modes `archive`, `resume`).
+TEST INFRASTRUCTURE: the checker is the UNMODIFIED reference (oracle/_ref/refdump, modes `archive` and `resume`), through
+what it computed on these scenarios (tests/refpin.py, tests/golden/reference/): its own archive file, its runs after
+loading that file and after loading the files this engine writes.
 
 What "equal" means here.  The reference's own file round trip is lossy: its JSON parser (rapidjson without
 kParseFullPrecisionFlag) returns some 17-digit numbers one ulp off, so an engine that loads a file does NOT continue the
@@ -17,8 +19,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 from oracle import harness as H   # noqa: E402
+import refpin   # noqa: E402
 
 STATE_FIELDS = ("flow", "cnt", "priority", "drivable", "dis", "speed", "leader_flow", "leader_cnt", "blocker_flow", "blocker_cnt", "gap")
+FOLLOW_PARTS = ("vehicle_count", "lane_count", "lane_waiting", "state")   # refpin parts of what follow() compares
 
 
 def compare_archives(ours: dict, ref: dict):
@@ -45,62 +49,58 @@ def compare_archives(ours: dict, ref: dict):
     return checked
 
 
-def follow(eng, states, tag):
-    """`eng` steps along the reference's dumped states: every running vehicle equal in every field."""
+def follow(eng, pin, tag):
+    """`eng` steps along the reference's pinned states: vehicle count, per-lane counts and waiting counts, and every
+    running vehicle in every field of STATE_FIELDS, every step."""
+    f = refpin.Follow(pin, tag=tag)
     g = None
-    for st in states:
-        eng.next_step()
-        assert eng.vehicle_count() == st.vehicle_count, (tag, st.step)
-        assert np.array_equal(eng.lane_vehicle_count(), st.lane_count), (tag, st.step)
-        assert np.array_equal(eng.lane_waiting_count(), st.lane_waiting), (tag, st.step)
-        g = np.sort(eng.debug_vehicles(), order=["flow", "cnt"])
-        o = np.sort(st.vehicles, order=["flow", "cnt"])
-        assert len(g) == len(o), (tag, st.step)
-        for f in STATE_FIELDS:
-            assert np.array_equal(g[f], o[f]), (tag, st.step, f)
+    for a, b in pin["steps"]:
+        for s in range(a, b + 1):
+            eng.next_step()
+            st = H.StepState()
+            st.vehicle_count = eng.vehicle_count()
+            st.lane_count, st.lane_waiting = eng.lane_vehicle_count(), eng.lane_waiting_count()
+            st.vehicles = g = eng.debug_vehicles()
+            f.add(s, st)
+    f.finish()
     return g
 
 
-def check_json_interchange(make_engine, cfg: str, tmp: str, n0: int, n1: int):
-    """Both directions at step `n0`, followed for `n1` steps:
-    (1) this engine's dump equals the reference's own dump field by field, and the reference loads it and then moves as it
-        does from its own file; (2) this engine loads the reference's file -- over an unrelated state -- and then moves
-        exactly as the reference does from that file, travel-time statistics included; (3) the file written here loads back
-        here to the same trajectory as (2)."""
+def check_json_interchange(make_engine, cfg: str, tmp: str):
+    """Both directions at step 120 of the dense 3x3 scenario, followed for 50 steps:
+    (1) this engine's dump equals the reference's own dump field by field, and it is the file the reference was seen to
+        load and then move exactly as from its own file; (2) this engine loads the reference's file -- over an unrelated
+        state -- and then moves exactly as the reference does from that file; (3) the file written here loads back here to
+        the same trajectory as (2), travel-time statistics included."""
+    import lzma
+    pin = refpin.load("archive_3x3_dense")
     ours_path, ref_path = os.path.join(tmp, "ours.json"), os.path.join(tmp, "ref.json")
+    with open(os.path.join(refpin.PINS, "archive_3x3_dense_step120.json.xz"), "rb") as f, open(ref_path, "wb") as g:
+        g.write(lzma.decompress(f.read()))
     eng = make_engine(cfg)
-    eng.next_step(n0)
+    eng.next_step(120)
     eng.dump(ours_path)
-    H.RefDump.archive(cfg, n0, ref_path)
     checked = compare_archives(json.load(open(ours_path)), json.load(open(ref_path)))
     assert checked > 20000
-    kw = dict(n_inter=eng.n_inter, n_drivables=eng.n_drivables)
-    from_ref = H.RefDump.resume(cfg, ref_path, n1, **kw)
-    from_ours = H.RefDump.resume(cfg, ours_path, n1, **kw)
-    for a, b in zip(from_ref, from_ours):
-        assert a.vehicle_count == b.vehicle_count and a.finished == b.finished and a.cum_travel_time == b.cum_travel_time
-        assert a.vehicles.tobytes() == b.vehicles.tobytes(), a.step
+    assert refpin.digest(open(ours_path, "rb").read()) == pin["ours_resumed_identically"], \
+        "the archive is not the file the reference was seen to resume like its own (re-record with tests/refpin.py archives)"
     # (2) the reference's file into an engine that is somewhere else entirely
     other = make_engine(cfg)
     other.next_step(17)
     other.load_from_file(ref_path)
-    g = follow(other, from_ref, "reference file")
+    g = follow(other, pin, "reference file")
     assert len(g) > 300
     # (3) our own file back into the first engine (it has moved on in the meantime)
     eng.next_step(5)
     eng.load_from_file(ours_path)
-    follow(eng, from_ref, "own file")
+    follow(eng, pin, "own file")
     assert eng.average_travel_time() == other.average_travel_time()
-    return from_ref
 
 
-def check_json_with_rl_phases(make_engine, cfg: str, tmp: str):
-    """rlTrafficLight mode, phases set right before the snapshot (not yet sent to the device when it is taken): the file
-    carries them, the reference resuming from it shows them and moves the vehicles as this engine does after loading the
-    same file."""
+def dump_with_rl_phases(eng, cfg: str, tmp: str):
+    """90 steps, then a phase for every signalised intersection and at once snapshot().dump("rl.json")."""
     roadnet = json.load(open(json.load(open(cfg))["dir"] + json.load(open(cfg))["roadnetFile"]))
     real = [k for k, i in enumerate(roadnet["intersections"]) if not i["virtual"]]
-    eng = make_engine(cfg)
     eng.next_step(90)
     want = {k: (3 * n + 1) % 8 for n, k in enumerate(real)}
     for k, ph in want.items():
@@ -111,11 +111,21 @@ def check_json_with_rl_phases(make_engine, cfg: str, tmp: str):
     assert doc["step"] == 90 and doc["activeVehicleCount"] == eng.vehicle_count()
     for k, ph in want.items():
         assert doc["trafficLights"][roadnet["intersections"][k]["id"]]["curPhaseIndex"] == ph
-    ref = H.RefDump.resume(cfg, path, 40, n_inter=eng.n_inter, n_drivables=eng.n_drivables)
-    assert [int(p) for p in ref[-1].phases if p >= 0] == [want[k] for k in real]
+    return path, [want[k] for k in real]
+
+
+def check_json_with_rl_phases(make_engine, cfg: str, tmp: str):
+    """rlTrafficLight mode, phases set right before the snapshot (not yet sent to the device when it is taken): the file
+    carries them, the reference resuming from it showed them and moved the vehicles as this engine does after loading the
+    same file."""
+    pin = refpin.load("archive_rl_6x6")
+    path, want = dump_with_rl_phases(make_engine(cfg), cfg, tmp)
+    assert refpin.digest(open(path, "rb").read()) == pin["ours"], \
+        "the archive is not the file the reference was seen to resume (re-record with tests/refpin.py archives)"
+    assert pin["phases"] == want
     other = make_engine(cfg)
     other.load_from_file(path)
-    follow(other, ref, "rl file")
+    follow(other, pin, "rl file")
 
 
 def check_reference_disk_io_tests(make_engine, cfg: str, tmp: str, record):

@@ -6,14 +6,14 @@
 Every rank steps its strip of ONE simulation (peer-memory seam exchange, or NCCL send/recv with
 CITYFLOW_B200_SHARD_TRANSPORT=nccl); the engine's COLLECTIVE observations -- get_vehicle_count() every 5 steps,
 get_lane_vehicle_count() and get_lane_waiting_vehicle_count() every `every` steps -- are compared on rank 0 with the
-unmodified reference (oracle/_ref/refdump counts, thread_num = host cores) run on the same scenario beforehand."""
+unmodified reference (oracle/_ref/refdump counts, thread_num = host cores) on the same scenario, through its pinned results
+(tests/refpin.py shard_runs)."""
 import json
 import os
 import sys
 import tempfile
 import time
 
-import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -21,6 +21,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import cityflow_b200  # noqa: E402
 from cityflow_b200 import scenario  # noqa: E402
+import refpin  # noqa: E402
 
 
 def main():
@@ -35,10 +36,7 @@ def main():
     cfg = scenario.make_grid_scenario(d, rows, cols, dense=dict(frac=frac, interval=interval, seed=seed, fleet_spread=spread), name="sh")
     ref = None
     if rank == 0:
-        from oracle import harness as H
-        t0 = time.time()
-        ref = H.RefDump.counts(cfg, steps, os.cpu_count() or 8, every)
-        print("reference: %d steps of %dx%d in %.1f s, %d vehicles at the end" % (steps, rows, cols, time.time() - t0, ref["vehicle_count"][-1]), flush=True)
+        ref = refpin.load("shard_runs")[refpin.shard_run_key(a)]
     dist.barrier()
     ids = [cityflow_b200.nccl_unique_id() if rank == 0 else None]
     dist.broadcast_object_list(ids, src=0)
@@ -52,18 +50,17 @@ def main():
         t_step += time.perf_counter() - t0
         if s % 5 == 0 or s == steps:
             n = eng.get_vehicle_count()                      # collective
-            if ref is not None and n != int(ref["vehicle_count"][s - 1]):
-                bad.append("step %d: vehicle count %d, reference %d" % (s, n, int(ref["vehicle_count"][s - 1])))
+            if ref is not None and n != ref["vehicle_count"][str(s)]:
+                bad.append("step %d: vehicle count %d, reference %d" % (s, n, ref["vehicle_count"][str(s)]))
         if s % every == 0 or s == steps:
             lanes = eng.get_lane_vehicle_count()            # collective
             wait = eng.get_lane_waiting_vehicle_count()     # collective
             if ref is not None:
-                rc, rw, _ = ref["dumps"][s]
-                mine = np.array([lanes[k] for k in lane_ids]), np.array([wait[k] for k in lane_ids])
-                if not np.array_equal(mine[0], rc):
-                    bad.append("step %d: %d lane counts differ" % (s, int((mine[0] != rc).sum())))
-                if not np.array_equal(mine[1], rw):
-                    bad.append("step %d: %d lane waiting counts differ" % (s, int((mine[1] != rw).sum())))
+                want = ref["lanes"][str(s)]
+                if refpin.lane_digest([lanes[k] for k in lane_ids]) != want["lane_count"]:
+                    bad.append("step %d: lane counts differ" % s)
+                if refpin.lane_digest([wait[k] for k in lane_ids]) != want["lane_waiting"]:
+                    bad.append("step %d: lane waiting counts differ" % s)
         if len(bad) > 6:
             break
     t = torch.tensor([eng.tie_count(), len(bad)], device="cuda", dtype=torch.int64)

@@ -1,6 +1,6 @@
 """GPU parity tests proper: the CUDA path, called through the C-ABI (ctypes), against the
-checkers on identical seeded inputs -- the compiled unmodified reference (oracle/_ref/refdump)
-when it travelled to this box, and the CPU restatement (oracle/cityflow_oracle.cpp).
+checkers on identical seeded inputs -- the compiled unmodified reference (oracle/_ref/refdump),
+through its pinned results (tests/refpin.py), and the CPU restatement (oracle/cityflow_oracle.cpp).
 
 Bar (BASELINE.json north_star): per-lane vehicle counts bit-exact every step, per-vehicle speeds
 within 1e-6.  What is asserted here is stronger: every running vehicle's (drivable, distance,
@@ -9,6 +9,7 @@ speed, leader, gap, blocker, enterLaneLinkTime) is bit-equal every step.
 import numpy as np
 import pytest
 
+import refpin
 from oracle import harness as H
 
 pytestmark = pytest.mark.gpu
@@ -92,24 +93,17 @@ def test_rl_phases_vs_port(cfg_6x6_rl):
             assert not bad, "step %d: %s" % (s, "; ".join(bad[:6]))
 
 
-@pytest.mark.skipif(not H.have_ref(), reason="compiled reference (oracle/_ref) not present")
 def test_6x6_dense_vs_compiled_reference(cfg_6x6_dense):
     from cityflow_b200.capi import CEngine
     eng = CEngine(cfg_6x6_dense)
-    steps, every = 800, 20
-    ref = H.RefDump.run(cfg_6x6_dense, steps, 1, every, n_inter=eng.n_inter, n_drivables=eng.n_drivables)
-    k = 0
-    for s in range(1, steps + 1):
-        eng.next_step()
-        if s % every == 0 or s == steps:
-            st = ref[k]
-            k += 1
-            assert st.step == s
-            st.lane_queue = None
-            st.phases = None
-            st.order = None
-            bad = H.compare_states(_relax(st), _gpu_state(eng, s))
-            assert not bad, "step %d: %s" % (s, "; ".join(bad[:6]))
+    pin = refpin.load("dense_6x6")
+    f = refpin.Follow(pin, parts=refpin.GPU, tag="6x6 dense")
+    done = 0
+    for _, step in pin["steps"]:        # every 20th step of 800
+        eng.next_step(step - done)
+        done = step
+        f.add(done, _gpu_state(eng, done))
+    f.finish()
 
 
 def test_reset_determinism(cfg_3x3_dense):
@@ -476,24 +470,11 @@ def test_lane_change_statistics_vs_unmodified_reference(tmp_path):
     """laneChange=true against the UNMODIFIED reference.  Its lane-change schedule follows heap addresses (the order of
     a std::set<Vehicle*>), so only aggregates can agree: vehicles that finished, lane changes started, mean speed, running
     vehicles -- same tolerances as the restatement's own comparison (tests/test_cpu.py)."""
-    if not H.have_ref():
-        pytest.skip("oracle/_ref was not built")
     from cityflow_b200 import scenario
     from cityflow_b200.capi import CEngine
     cfg = scenario.make_grid_scenario(str(tmp_path), 5, 5, dense=dict(frac=1.0, interval=2.0, seed=11), name="lcstat", lane_change=True)
     eng = CEngine(cfg)
-    ref = H.RefDump.runlc(cfg, 800, 1, n_inter=eng.n_inter, n_drivables=eng.n_drivables, patched=False)
-
-    def summary(states):
-        started, seen, speed = 0, set(), []
-        for st in states:
-            sh = st.vehicles["priority"][st.vehicles["partner_type"] == 2]
-            started += len(set(sh.tolist()) - seen)
-            seen |= set(sh.tolist())
-            speed.append(float(st.vehicles["speed"].mean()))
-        return dict(finished=states[-1].finished, started=started, speed=float(np.mean(speed[200:])), vehicles=len(states[-1].vehicles))
-
-    a, b = summary(ref), summary(_lc_gpu_states(eng, 800))
+    a, b = refpin.load("lc_statistics"), refpin.lc_summary(_lc_gpu_states(eng, 800))
     assert a["started"] > 200 and b["started"] > 200, (a, b)
     for k, tol in (("finished", 0.03), ("started", 0.15), ("speed", 0.03), ("vehicles", 0.03)):
         assert abs(a[k] - b[k]) <= tol * a[k], (k, a, b)
@@ -547,22 +528,17 @@ def test_fuzzed_irregular_networks_vs_port(seed, tmp_path):
 def test_fuzzed_network_vs_compiled_reference(tmp_path):
     """The same kind of network straight against the UNMODIFIED reference (oracle/_ref/refdump): the restatement shares the
     product's loader, the compiled reference does not -- a loader / routing bug cannot hide behind it here."""
-    if not H.have_ref():
-        pytest.skip("oracle/_ref was not built")
-    import randnet
-    from cityflow_b200 import scenario
     from cityflow_b200.capi import CEngine
-    net = randnet.random_roadnet(4, rows=3, cols=4)
-    flows = randnet.random_flows(net, 104, n_flows=70)
-    cfg = scenario.write_scenario(str(tmp_path), net, flows, seed=4, interval=1.0, name="gref")
+    cfg = refpin.random_network_config(str(tmp_path), 4, 1.0, "gref", n_flows=70, rows=3, cols=4)
     eng = CEngine(cfg)
-    ref = H.RefDump.run(cfg, 500, threads=2, every=10, n_inter=eng.n_inter, n_drivables=eng.n_drivables)
+    pin = refpin.load("fuzzed_network_4")     # reference with thread_num=2, every 10th step of 500
+    f = refpin.Follow(pin, parts=refpin.GPU, tag="fuzzed network 4")
     done = 0
-    for st in ref:
-        eng.next_step(st.step - done)
-        done = st.step
-        bad = H.compare_states(_relax(st), _gpu_state(eng, st.step), check_order=False)
-        assert not bad, "step %d: %s" % (st.step, "; ".join(bad[:6]))
+    for _, step in pin["steps"]:
+        eng.next_step(step - done)
+        done = step
+        f.add(done, _gpu_state(eng, done))
+    f.finish()
     assert eng.tie_count() == 0
 
 
@@ -605,30 +581,30 @@ def test_30x30_through_the_bench_window_vs_compiled_reference(scenario_dir):
     reference -- vehicle count after every step, per-lane counts, per-lane waiting counts (speed < 0.1) and per-lane speed
     sums (within 1e-6 per vehicle) every 50 steps and at steps 1200, 1210, 1220, 1230 (the vehicle count at every step of
     the window 1200..1230)."""
-    if not H.have_ref():
-        pytest.skip("oracle/_ref was not built")
-    import os
     from cityflow_b200 import scenario
     from cityflow_b200.capi import CEngine
     cfg = scenario.make_grid_scenario(scenario_dir, 30, 30, name="g30w", dense=dict(frac=0.5, interval=10.0, seed=1, fleet_spread=0.02))
-    ref = H.RefDump.counts(cfg, 1230, os.cpu_count() or 8, 10)
+    ref = refpin.load("bench_window_30x30")   # the reference with thread_num = host cores
+    assert ref["lanes"].keys() == {str(s) for s in refpin.bench_window_steps()}
     eng = CEngine(cfg)
     for s in range(1, 1231):
         eng.next_step()
         if s >= 1200 or s % 5 == 0:
-            assert eng.vehicle_count() == int(ref["vehicle_count"][s - 1]), s
-        if s % 10 or (s % 50 and s < 1200):
+            assert eng.vehicle_count() == ref["vehicle_count"][str(s)], s
+        if str(s) not in ref["lanes"]:
             continue
-        rc, rw, rs = ref["dumps"][s]
-        assert eng.vehicle_count() == int(ref["vehicle_count"][s - 1]), s
         mc, mw = eng.lane_vehicle_count(), eng.lane_waiting_count()
-        assert np.array_equal(mc, rc), "step %d: %d lane counts differ" % (s, int((mc != rc).sum()))
-        assert np.array_equal(mw, rw), "step %d: %d lane waiting counts differ" % (s, int((mw != rw).sum()))
-    # per-vehicle speeds at the end, through the per-lane speed sums (bar: 1e-6 per vehicle; the sums differ by summation order only)
+        assert refpin.lane_digest(mc) == ref["lanes"][str(s)]["lane_count"], "step %d: lane counts differ" % s
+        assert refpin.lane_digest(mw) == ref["lanes"][str(s)]["lane_waiting"], "step %d: lane waiting counts differ" % s
+    # per-vehicle speeds at the end, through the per-lane speed sums (bar: 1e-6 per vehicle; the sums differ by summation order
+    # only): on a seeded sample of 512 lanes, and in total
     v = eng.debug_vehicles()
     on = v[v["drivable"] < eng.n_lanes]
     mine = np.bincount(on["drivable"], weights=on["speed"], minlength=eng.n_lanes)
-    assert np.all(np.abs(mine - rs) <= 1e-6 * np.maximum(mc, 1)), "per-lane speed sums differ"
+    pick, rs = np.array(ref["speed_sum_lanes"]), np.array(ref["speed_sum"])
+    assert eng.n_lanes == ref["n_lanes"] and int(mc.sum()) == ref["vehicles_on_lanes"]
+    assert np.all(np.abs(mine[pick] - rs) <= 1e-6 * np.maximum(mc[pick], 1)), "per-lane speed sums differ"
+    assert abs(mine.sum() - ref["speed_sum_total"]) <= 1e-6 * int(mc.sum()), "speed sum over all lanes differs"
     assert eng.vehicle_count() > 120000
     assert eng.tie_count() == 0   # (the bench fleet: no entrant tie, so the reference's result is defined -- bench.py FLEET_SPREAD)
 

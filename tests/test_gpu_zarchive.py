@@ -1,5 +1,6 @@
 """GPU test of the archive in the reference's JSON schema (SURVEY.md section 8 row f2): Archive.dump("x.json") and
-load_from_file() interchange with the unmodified reference (oracle/_ref/refdump `archive` / `resume`) in both directions.
+load_from_file() interchange with the unmodified reference (oracle/_ref/refdump `archive` / `resume`, pinned) in both
+directions.
 The checks (tests/archive_checks.py), the host logic and the image codec are the ones tests/test_cpu.py runs over the
 emulated device; here the image goes to / comes from the real device through DeviceSim::snapshotToHost /
 snapshotFromHost + restore, the calls the binary archive uses.
@@ -21,7 +22,7 @@ def _engine(cfg):
 
 
 def test_json_archive_interchanges_with_the_reference(cfg_3x3_dense, tmp_path):
-    archive_checks.check_json_interchange(_engine, cfg_3x3_dense, str(tmp_path), 120, 50)
+    archive_checks.check_json_interchange(_engine, cfg_3x3_dense, str(tmp_path))
 
 
 def test_json_archive_with_rl_phases(cfg_6x6_rl, tmp_path):
